@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the CAVI sweep hot path: SNP x trait updates/s (BASELINE.json's metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--config C2] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--config C2] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one full VB iteration of the BASELINE config as `atlasqtl()` would run it: the host
 q-/p-sized algebra, the fused sweep kernel (coreDualLoop + its reductions), the row sums of Z, the
@@ -16,6 +16,12 @@ all-reduce (N > 1) and the table refresh (+ ELBO part once annealing is over).
 
 `--impl reference` times the reference's own coreDualLoop (oracle/_ref: src/coreLoop.cpp compiled
 unmodified) on the host cores, on a bounded sample of the same workload.
+
+`--dump-outputs DIR` writes, after the timed steps, what the timed path returned after its last step as DIR/<name>.npy
+(float64): gam_vb, beta_vb, theta_vb, zeta_vb (the reference arm: its gam_vb, mu_beta_vb, beta_vb).  The inputs are
+seeded, so two builds run with the same arguments can be compared output for output.  A p x q output too large for
+DUMP_BYTES in all is written as a fixed, seeded sample of its entries, <name>_sample.npy, with their column-major
+positions in pq_sample_index.npy.  With N > 1 ranks each rank writes its own trait slab, with the suffix .rank<r>.
 """
 import argparse
 import json
@@ -62,6 +68,29 @@ FP64_PEAK_TFLOPS = 37.05  # measured DMMA m8n8k4 peak on this pool's B200 (profi
 
 def log(*a):
     print(*a, file=sys.stderr, flush=True)
+
+
+DUMP_BYTES = 64 << 20       # --dump-outputs: at most this much in all (over all ranks)
+DUMP_SAMPLE = 1 << 21       # entries kept of each large p x q output (split over the ranks)
+
+
+def dump_outputs(dirname, arrays, rank=0, world=1):
+    """Write `arrays` (name -> vector or p x q matrix) as float64 .npy files under `dirname` (see the module doc)."""
+    os.makedirs(dirname, exist_ok=True)
+    suffix = f".rank{rank}" if world > 1 else ""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    mats = {k: v for k, v in arrays.items() if v.ndim == 2}
+    if world * sum(v.nbytes for v in arrays.values()) > DUMP_BYTES and mats:
+        shape = next(iter(mats.values())).shape
+        size = shape[0] * shape[1]
+        idx = np.sort(np.random.default_rng([123, rank]).choice(size, min(size, DUMP_SAMPLE // world), replace=False))
+        np.save(os.path.join(dirname, f"pq_sample_index{suffix}.npy"), idx.astype(np.float64))
+        for k, v in mats.items():
+            assert v.shape == shape
+            arrays.pop(k)
+            arrays[k + "_sample"] = v.ravel(order="F")[idx]
+    for k, v in arrays.items():
+        np.save(os.path.join(dirname, f"{k}{suffix}.npy"), v)
 
 
 # ----------------------------------------------------------------------------- workload
@@ -253,6 +282,7 @@ def reference_sample(cfg, X, Y, hyper, init, p_s=8192, traits_per_thread=1, thre
     ms = 1e3 * float(np.mean(times))
     value = p_s * q_s / (ms / 1e3)
     return dict(value=value, unit="SNPxtrait updates/s", cores=len(ranges), kind=kind, ms_per_step=ms,
+                outputs=dict(gam_vb=gam, mu_beta_vb=mu, beta_vb=beta),
                 sample=f"coreDualLoop (dual/Gram form, as the reference runs it), n={n}, first {p_s} of {p} SNPs x "
                        f"{q_s} traits, {len(ranges)} host threads on disjoint sample_q ranges; Gram set-up {setup_s:.1f} s "
                        f"not timed; dual-form cost per update grows with p, so at the full p this is ~{p_s / p:.3g}x",
@@ -308,7 +338,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--na-frac", type=float, default=0.0,
                     help="fraction of missing responses (NaN in Y): times the coreDualMisLoop path instead of coreDualLoop")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed path computed in its last step to DIR/<name>.npy (see the module doc)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     # stdout carries the ONE JSON line and nothing else: whatever libraries print there (NCCL's version banner, ...) is
     # sent to stderr by pointing fd 1 at fd 2 for the run; the line itself goes to the saved descriptor
     sys.stdout.flush()
@@ -321,7 +355,7 @@ def main():
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
-    W, K = max(args.warmup, 0), max(args.steps, 1)
+    W, K = args.warmup, args.steps
 
     from atlasqtl_b200 import synthetic
     from atlasqtl_b200.dist import slab_bounds
@@ -344,6 +378,8 @@ def main():
         ncpu = os.cpu_count() or 1
         ws = make_workload(args.config, 0, min(q, 4 * ncpu))
         res = reference_sample(*ws, steps=K, warmup=W)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, res["outputs"])
         # the reference's dual form needs the p x p Gram matrix (20 GB at C2) and O(p) work per update: it is timed on a
         # bounded SAMPLE of the workload, and the line says so where the config is named
         config["workload"] += f" -- REFERENCE ARM TIMES A SAMPLE: {res['sample']}"
@@ -446,10 +482,13 @@ def main():
         Xarg = X
     log(f"[rank {rank}] context created in {time.time() - t_up:.1f} s")
     try:
-        core.atlasqtl_global_local_core_(Y, Xarg, q, anneal, 1, 1e-300, W + K, 0, hyper, init, debug=False, comm=comm,
-                                         slab=(k0, k1), ctx=ctx, trace=trace, iter_hook=hook, release_x=True)
+        result = core.atlasqtl_global_local_core_(Y, Xarg, q, anneal, 1, 1e-300, W + K, 0, hyper, init, debug=False,
+                                                  comm=comm, slab=(k0, k1), ctx=ctx, trace=trace, iter_hook=hook,
+                                                  release_x=True)
         clocks = sampler.stop() if rank == 0 else None
         timed = [r for r in trace if W < r["it"] <= W + K]
+        if len(timed) != K or "t1" not in marks:
+            raise SystemExit(f"the run stopped after {result['it']} of {W + K} iterations: {len(timed)} of {K} steps timed")
         seg_keys = list(timed[0].get("host_ms", {})) if timed else []
         host_ms = np.array([np.mean([r["host_ms"].get(k, 0.0) for r in timed]) for k in seg_keys])
         dev_ms = sum(r["sweep_ms"] + r["rows_ms"] + r["tables_ms"] for r in timed)
@@ -480,6 +519,9 @@ def main():
                          "different GPU counts must agree to ~1e-10 relative"}
     finally:
         ctx.close()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: result[k] for k in ("gam_vb", "beta_vb", "zeta_vb")}
+                     | ({"theta_vb": result["theta_vb"]} if rank == 0 else {}), rank, world)
     if rank != 0:
         if world > 1:
             torch.distributed.destroy_process_group()

@@ -84,9 +84,18 @@ def run_core(it, X, Y, hyper, init, anneal, thinned, tol, maxit=1000):
     return res
 
 
+MAX_FILE_BYTES = 1_000_000
+SPLIT_KEYS = ("init_gam_vb", "init_mu_beta_vb")
+
+
 def save(name, **arrays):
     dest = os.path.join(HERE, name)
     np.savez_compressed(dest, **arrays)
+    if name.startswith("rlite_core_") and os.path.getsize(dest) > MAX_FILE_BYTES:
+        # keep every file under 1 MB: the initial p x q matrices go to rlite_init_<case>.npz (tests/rlite_cases.py
+        # merges it back)
+        save("rlite_init_" + name[len("rlite_core_"):], **{k: arrays[k] for k in SPLIT_KEYS})
+        np.savez_compressed(dest, **{k: v for k, v in arrays.items() if k not in SPLIT_KEYS})
     print(f"wrote {dest} ({os.path.getsize(dest) / 1024:.0f} KiB)", flush=True)
 
 

@@ -1,9 +1,11 @@
 """CPU tests of the host driver (atlasqtl_b200.core) with the oracle-backed test double in place of the
 CUDA context: the re-expression of the R updates through per-trait / per-SNP sums must reproduce the
-line-by-line restatement of the R loop (oracle/vb_oracle.py), iteration by iteration."""
+line-by-line restatement of the R loop (oracle/vb_oracle.py), iteration by iteration; with the reference's own
+sweep, its stored runs (tests/reference_runs.py)."""
 import numpy as np
 import pytest
 
+import reference_runs
 from atlasqtl_b200 import core
 from fake_context import OracleSweepContext
 from oracle import vb_oracle
@@ -12,35 +14,39 @@ from problems import make_problem
 
 @pytest.mark.parametrize("anneal", [None, (1, 2, 10), (2, 3, 5), (3, 2, 4)])
 def test_host_loop_matches_restated_r_loop(oracle_built, anneal):
-    X, Y, hyper, init = make_problem(100, 75, 20, p_act=10, q_act=20, maf=0.2, p0=(5, 25))
+    X, Y, hyper, init = reference_runs.host_problem()
     q = Y.shape[1]
-    tr_o, tr_c = [], []
-    ref = vb_oracle.atlasqtl_global_local_core_(Y, X, q, anneal, 1, 0.1, 1000, hyper, init, sweep="reference",
-                                                trace=tr_o)
+    tr_c = []
+    ref = reference_runs.load("host", anneal)   # the restated R loop with the reference's own sweep
+    tr_o = ref["trace"]
+    np.testing.assert_allclose(reference_runs.in_check(X, Y, init), ref["in_check"], rtol=1e-12)
     out = core.atlasqtl_global_local_core_(Y, X, q, anneal, 1, 0.1, 1000, 0, hyper, init, debug=True,
                                            context_factory=lambda X_, Y_: OracleSweepContext(X_, Y_), trace=tr_c)
     assert ref["converged"] and out["converged"]
     assert out["it"] == ref["it"]
+    assert len(tr_o) == len(tr_c)
     for a, b in zip(tr_o, tr_c):
         assert a["it"] == b["it"] and abs(a["c"] - b["c"]) < 1e-15
         assert (a["lb"] is None) == (b["lb"] is None)
         if a["lb"] is not None:
             assert abs(a["lb"] - b["lb"]) <= 1e-10 * abs(a["lb"])
-    assert np.abs(out["gam_vb"] - ref["gam_vb"]).max() <= 1e-10
+    assert np.abs(ref["pick"](out["gam_vb"]) - ref["gam_vb"]).max() <= 1e-10
+    assert np.array_equal(out["gam_vb"] > 0.5, ref["sel"])
     np.testing.assert_allclose(out["theta_vb"], ref["theta_vb"], rtol=1e-9, atol=1e-10)
     np.testing.assert_allclose(out["zeta_vb"], ref["zeta_vb"], rtol=1e-9, atol=1e-10)
 
 
 def test_order_fn_is_honoured(oracle_built):
-    X, Y, hyper, init = make_problem(100, 60, 12, p_act=6, q_act=12)
-    q, p = Y.shape[1], X.shape[1]
-    perm = lambda it, p_: np.random.default_rng(it).permutation(p_).astype(np.int32)
-    ref = vb_oracle.atlasqtl_global_local_core_(Y, X, q, None, 1, 0.1, 50, hyper, init, sweep="reference", perm_fn=perm)
-    out = core.atlasqtl_global_local_core_(Y, X, q, None, 1, 0.1, 50, 0, hyper, init, debug=True, order_fn=perm,
+    X, Y, hyper, init = reference_runs.order_problem()
+    q = Y.shape[1]
+    ref = reference_runs.load("order", "perm")   # the restated R loop with the reference's own sweep, shuffled order
+    np.testing.assert_allclose(reference_runs.in_check(X, Y, init), ref["in_check"], rtol=1e-12)
+    out = core.atlasqtl_global_local_core_(Y, X, q, None, 1, 0.1, 50, 0, hyper, init, debug=True,
+                                           order_fn=reference_runs.order_perm,
                                            context_factory=lambda X_, Y_: OracleSweepContext(X_, Y_))
     assert out["it"] == ref["it"]
-    assert np.abs(out["gam_vb"] - ref["gam_vb"]).max() <= 1e-10
-    ident = vb_oracle.atlasqtl_global_local_core_(Y, X, q, None, 1, 0.1, 50, hyper, init, sweep="reference")
+    assert np.abs(ref["pick"](out["gam_vb"]) - ref["gam_vb"]).max() <= 1e-10
+    ident = reference_runs.load("order", "identity")
     assert np.abs(ident["gam_vb"] - ref["gam_vb"]).max() > 1e-8  # the order really changes the trajectory
 
 

@@ -1,8 +1,9 @@
 """GPU: full VB runs through the C ABI against the restated R loop on the CPU oracle
-(sweep = the reference's own coreLoop.cpp where its p x p inputs are feasible)."""
+(sweep = the reference's own coreLoop.cpp where its p x p inputs are feasible: its stored runs, tests/reference_runs.py)."""
 import numpy as np
 import pytest
 
+import reference_runs
 from problems import make_problem
 
 pytestmark = pytest.mark.gpu
@@ -21,17 +22,24 @@ def test_trajectory_parity(oracle_built, n, p, q, anneal, form):
     from oracle import vb_oracle
     X, Y, hyper, init = make_problem(n, p, q)
     q = Y.shape[1]
-    tr_o, tr_g = [], []
-    ref = vb_oracle.atlasqtl_global_local_core_(Y, X, q, anneal, 1, 0.1, 1000, hyper, init, sweep=form, trace=tr_o,
-                                                nthreads=4)
+    tr_g = []
+    if form == "reference":
+        ref = reference_runs.load("full", n, p, q, anneal)
+        np.testing.assert_allclose(reference_runs.in_check(X, Y, init), ref["in_check"], rtol=1e-12)
+    else:
+        tr_o = []
+        run = vb_oracle.atlasqtl_global_local_core_(Y, X, q, anneal, 1, 0.1, 1000, hyper, init, sweep=form, trace=tr_o,
+                                                    nthreads=4)
+        ref = reference_runs.with_views(reference_runs.run_summary(run, tr_o, sample=False))
     out = core.atlasqtl_global_local_core_(Y, X, q, anneal, 1, 0.1, 1000, 0, hyper, init, debug=True, trace=tr_g)
     assert out["converged"] and ref["converged"]
     assert out["it"] == ref["it"]
-    for a, b in zip(tr_o, tr_g):
+    for a, b in zip(ref["trace"], tr_g):
         if a["lb"] is not None:
             assert abs(a["lb"] - b["lb"]) <= 1e-10 * abs(a["lb"]), (a["it"], a["lb"], b["lb"])
-    assert np.abs(out["gam_vb"] - ref["gam_vb"]).max() <= 1e-8
-    assert np.abs(out["beta_vb"] - ref["beta_vb"]).max() <= 1e-8
+    pick = ref["pick"]   # every entry, or the stored sample of the reference's run
+    assert np.abs(pick(out["gam_vb"]) - ref["gam_vb"]).max() <= 1e-8
+    assert np.abs(pick(out["beta_vb"]) - ref["beta_vb"]).max() <= 1e-8
     # integer outputs: selection sets must be identical
-    assert np.array_equal(out["gam_vb"] > 0.5, ref["gam_vb"] > 0.5)
-    assert np.array_equal(summarise.assign_bFDR(out["gam_vb"]) < 0.05, vb_oracle.assign_bFDR(ref["gam_vb"]) < 0.05)
+    assert np.array_equal(out["gam_vb"] > 0.5, ref["sel"])
+    assert np.array_equal(summarise.assign_bFDR(out["gam_vb"]) < 0.05, ref["sel_bfdr"])

@@ -37,21 +37,13 @@ def test_logistic_neg_full_range(variant):
 def test_sweep_with_saturated_probabilities(oracle_built):
     """theta + zeta driven to +-30 and huge effects: gam_vb saturates at 0 and 1 (logistic arguments beyond +-700);
     the CUDA sweep must agree with the reference's own loop there too."""
+    import reference_runs
     from atlasqtl_b200.device import SweepContext
-    from problems import make_problem, sweep_inputs
-    from scipy import special as sp
-    from test_gpu_sweep import oracle_sweep
-    X, Y, hyper, init = make_problem(120, 60, 24)
-    p, q = X.shape[1], Y.shape[1]
-    Y = np.asfortranarray(Y * 40.0)   # strong signals: mu^2 / (2 sig2_beta) in the thousands
-    si = sweep_inputs(X, Y, init, c=1.0)
-    rng = np.random.default_rng(3)
-    si["theta"] = rng.choice([-30.0, 0.0, 9.0], size=p)
-    si["zeta"] = rng.choice([-8.0, 0.0, 3.0], size=q)
-    u = si["theta"][:, None] + si["zeta"][None, :]
-    si["log_Phi"], si["log_1_min_Phi"] = np.asfortranarray(sp.log_ndtr(u)), np.asfortranarray(sp.log_ndtr(-u))
-    order = np.arange(p, dtype=np.int32)
-    g_ref, m_ref, b_ref, R_ref = oracle_sweep(oracle_built, X, Y, si, order, "reference")
+    # strong signals (Y scaled by 40: mu^2 / (2 sig2_beta) in the thousands), theta + zeta at +-30 / +-8
+    X, Y, si, _ = reference_runs.saturated_inputs()
+    ref = reference_runs.load("saturated")   # the reference's own loop on these inputs
+    np.testing.assert_allclose(reference_runs.in_check(X, Y), ref["in_check"], rtol=1e-12)
+    pick, g_ref, b_ref = ref["pick"], ref["gam"], ref["beta"]
     assert (g_ref == 0).any() or (g_ref < 1e-300).any()
     assert (g_ref == 1).any()
     with SweepContext(X, Y) as ctx:
@@ -60,5 +52,5 @@ def test_sweep_with_saturated_probabilities(oracle_built):
         ctx.sweep(1.0, si["log_sig2_inv"], si["tau"], si["log_tau"], si["sig2_beta"])
         st = ctx.get_state()
     assert np.isfinite(st["gam_vb"]).all() and np.isfinite(st["mu_beta_vb"]).all()
-    assert np.abs(st["gam_vb"] - g_ref).max() <= 1e-9
-    assert np.abs(st["beta_vb"] - b_ref).max() <= 1e-9 * max(1.0, np.abs(b_ref).max())
+    assert np.abs(pick(st["gam_vb"]) - g_ref).max() <= 1e-9
+    assert np.abs(pick(st["beta_vb"]) - b_ref).max() <= 1e-9 * max(1.0, ref["beta_absmax"])

@@ -7,7 +7,7 @@ import numpy as np
 import pytest
 
 from problems import make_problem, sweep_inputs
-from test_gpu_sweep import oracle_sweep, zparts
+from reference_runs import oracle_sweep, zparts
 
 pytestmark = pytest.mark.gpu
 

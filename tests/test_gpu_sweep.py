@@ -1,47 +1,13 @@
 """GPU parity of one sweep through the C ABI against the CPU oracle (and, at dual-feasible sizes,
-against the reference's own coreLoop.cpp).  Tolerances: max|d gam_vb| <= 1e-8 (north_star), tighter in practice."""
+against the reference's own coreLoop.cpp: its stored outputs, tests/reference_runs.py).  Tolerances: max|d gam_vb| <= 1e-8
+(north_star), tighter in practice."""
 import numpy as np
 import pytest
 
+import reference_runs
 from problems import make_problem, sweep_inputs
 
 pytestmark = pytest.mark.gpu
-
-LOG_SQRT_2PI = 0.5 * np.log(2 * np.pi)
-
-
-def oracle_sweep(native, X, Y, si, order, form):
-    gam, mu = si["gam"].copy(order="F"), si["mu"].copy(order="F")
-    beta = np.asfortranarray(gam * mu)
-    q = Y.shape[1]
-    if form == "reference":
-        cp_X = np.asfortranarray(X.T @ X)
-        cp_Y_X = np.asfortranarray(Y.T @ X)
-        cbx = np.asfortranarray(cp_X @ beta)
-        native.core_dual_loop(cp_X, cp_Y_X, gam, si["log_Phi"], si["log_1_min_Phi"], si["log_sig2_inv"], si["log_tau"],
-                              beta, cbx, mu, si["sig2_beta"], si["tau"], order, np.arange(q, dtype=np.int32),
-                              c=si["c"], impl="reference")
-        R = np.asfortranarray(Y - X @ beta)
-    else:
-        R = native.residual(X, Y, beta)
-        xn = np.asfortranarray(np.sum(X ** 2, axis=0))
-        native.sweep_primal(X, xn, R, gam, si["log_Phi"], si["log_1_min_Phi"], si["log_sig2_inv"], si["log_tau"], beta,
-                            mu, si["sig2_beta"], si["tau"], order, c=si["c"], nthreads=4)
-    return gam, mu, beta, R
-
-
-def zparts(si, gam):
-    from scipy import special as sp
-    u = si["theta"][:, None] + si["zeta"][None, :]
-    sc = 1.0 if abs(si["c"] - 1) < 1.5e-8 else np.sqrt(si["c"])
-    U = sc * u
-    lp, lq = sp.log_ndtr(U), sp.log_ndtr(-U)
-    m1 = np.exp(-U ** 2 / 2 - LOG_SQRT_2PI - lp)
-    m1 = np.where(m1 < -U, -U, m1)
-    m0 = -np.exp(-U ** 2 / 2 - LOG_SQRT_2PI - lq)
-    m0 = np.where(m0 > -U, -U, m0)
-    zp = gam * (m1 - m0) + m0
-    return zp.sum(axis=0), zp.sum(axis=1)
 
 
 @pytest.mark.parametrize("n,p,q,c,form,shuffle", [
@@ -63,7 +29,13 @@ def test_single_sweep_parity(oracle_built, n, p, q, c, form, shuffle):
     p = X.shape[1]
     si = sweep_inputs(X, Y, init, c=c)
     order = (np.random.default_rng(5).permutation(p) if shuffle else np.arange(p)).astype(np.int32)
-    g_ref, m_ref, b_ref, R_ref = oracle_sweep(native, X, Y, si, order, form)
+    if form == "reference":
+        ref = reference_runs.load("sweep", n, p, q, c, shuffle)
+        np.testing.assert_allclose(reference_runs.in_check(X, Y, init), ref["in_check"], rtol=1e-12)
+    else:
+        ref = reference_runs.with_views(reference_runs.sweep_summary(
+            si, *reference_runs.oracle_sweep(native, X, Y, si, order, form), sample=False))
+    pick = ref["pick"]   # every entry, or the stored sample of the reference's sweep
 
     with SweepContext(X, Y) as ctx:
         ctx.set_order(order)
@@ -82,14 +54,13 @@ def test_single_sweep_parity(oracle_built, n, p, q, c, form, shuffle):
         R = ctx.get_residual()
         rows = ctx.rowsums_zpart()
 
-    assert np.abs(st["gam_vb"] - g_ref).max() <= 1e-9
-    assert np.abs(st["mu_beta_vb"] - m_ref).max() <= 1e-9 * max(1.0, np.abs(m_ref).max())
-    assert np.abs(st["beta_vb"] - b_ref).max() <= 1e-9
-    np.testing.assert_allclose(R, R_ref, atol=1e-9)
-    np.testing.assert_allclose(out["colsum_gam"], g_ref.sum(axis=0), rtol=1e-9, atol=1e-9)
-    np.testing.assert_allclose(out["colsum_beta2"], (b_ref ** 2).sum(axis=0), rtol=1e-9, atol=1e-9)
-    np.testing.assert_allclose(out["colsum_gam_mu2"], (g_ref * m_ref ** 2).sum(axis=0), rtol=1e-9, atol=1e-9)
-    np.testing.assert_allclose(out["resid_sq"], (R_ref ** 2).sum(axis=0), rtol=1e-9)
-    zc, zr = zparts(si, g_ref)
-    np.testing.assert_allclose(out["colsum_zpart"], zc, rtol=1e-9, atol=1e-8)
-    np.testing.assert_allclose(rows, zr, rtol=1e-9, atol=1e-8)
+    assert np.abs(pick(st["gam_vb"]) - ref["gam"]).max() <= 1e-9
+    assert np.abs(pick(st["mu_beta_vb"]) - ref["mu"]).max() <= 1e-9 * max(1.0, ref["mu_absmax"])
+    assert np.abs(pick(st["beta_vb"]) - ref["beta"]).max() <= 1e-9
+    np.testing.assert_allclose(ref["pick_R"](R), ref["R"], atol=1e-9)
+    np.testing.assert_allclose(out["colsum_gam"], ref["colsum_gam"], rtol=1e-9, atol=1e-9)
+    np.testing.assert_allclose(out["colsum_beta2"], ref["colsum_beta2"], rtol=1e-9, atol=1e-9)
+    np.testing.assert_allclose(out["colsum_gam_mu2"], ref["colsum_gam_mu2"], rtol=1e-9, atol=1e-9)
+    np.testing.assert_allclose(out["resid_sq"], ref["resid_sq"], rtol=1e-9)
+    np.testing.assert_allclose(out["colsum_zpart"], ref["colsum_zpart"], rtol=1e-9, atol=1e-8)
+    np.testing.assert_allclose(rows, ref["rowsum_zpart"], rtol=1e-9, atol=1e-8)
