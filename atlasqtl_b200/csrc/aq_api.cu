@@ -39,105 +39,55 @@ int fail(int code, const std::string& msg) {
         }                                                                                               \
     } while (0)
 
-// ---- kernel configurations (SweepCfg<MT, NT, clustered>): picked by n at aq_create time.
-// 14 MMA warps split a CTA's samples (112 NT of them); each holds MT 8-trait tiles: MT * NT * 2 accumulator doubles
-// (<= 40: the 16-warp CTA leaves 128 registers per thread).  n <= 1008: one CTA per trait tile.  n > 1008: a
-// thread-block cluster of 2 / 4 / 8 CTAs splits the samples (up to n = 7168).
-struct CfgInfo {
-    int id, n_pad, xs, kT, threads;   // n_pad: samples per CTA (slice), padded
-    size_t smem, tile_doubles;
-    int ncta;                         // CTAs per cluster (sample slices)
-};
-template <class C>
-CfgInfo info(int id, int ncta = 1) {
-    return CfgInfo{id, C::kNPad, C::kXS, C::kT, C::kThreads, C::kSmemBytes, C::kTileDoubles, ncta};
-}
-// traits / tile = 8 MT: 16, 24 or 32.  Beyond 16 the helper warp handles one trait per lane (no half-warp split), which the
+// ---- kernel configurations (SweepCfg<MT, NT, clustered, missing>): picked by n and q at aq_create time, and again by
+// aq_set_missing for the missing-response variant.  14 MMA warps split a CTA's samples (112 NT of them); each holds MT
+// 8-trait tiles: MT * NT * 2 accumulator doubles (<= 42: the 16-warp CTA leaves 128 registers per thread).  n <= 1008: one
+// CTA per trait tile.  n > 1008: a thread-block cluster of 2, 3, 4, 6 or 8 CTAs splits the samples (up to n = 7168).
+// Traits / tile = 8 MT: 16, 24 or 32.  Beyond 16 the helper warp handles one trait per lane (no half-warp split), which the
 // extra DSMEM hop of the clustered variant cannot afford at 7 sample tiles per warp.
 constexpr int mt_of_nt(int nt, bool cl) { return nt >= (cl ? 7 : 8) ? 2 : (nt >= 6 ? 3 : 4); }
-constexpr int kMaxNT = 9;    // single CTA: n <= 1008
-constexpr int kMaxNTCl = 8;  // clustered (the leader also buffers the followers' S tiles): n <= ncta * 896
 template <int NT, bool CL>
 using CfgOf = SweepCfg<mt_of_nt(NT, CL), NT, CL>;
-
-// id = nt (single CTA) or 100 + nt (clustered)
-template <int NT>
-bool pick_nt(int nt, bool cl, int ncta, CfgInfo* out) {
-    if (nt == NT) {
-        if (!cl) *out = info<CfgOf<NT, false>>(NT, 1);
-        else if constexpr (NT <= kMaxNTCl) *out = info<CfgOf<NT, true>>(100 + NT, ncta);
-        else return false;
-        return true;
-    }
-    if constexpr (NT < kMaxNT) return pick_nt<NT + 1>(nt, cl, ncta, out);
-    return false;
-}
-
-// ---- missing-response variants (SweepCfg<2, NT, clustered, true>, ids 1000 + ...): 16-trait tiles, and fewer sample
-// tiles per warp than the dense kernel so that the per-trait Gram band buffers (32 KB) fit beside the X tile ring:
-// NT <= 7 in one CTA (n <= 784), NT <= 6 in clusters of 2 / 4 / 6 / 8 CTAs (n <= 5376).
-constexpr int kMaxNTMis = 7, kMaxNTMisCl = 6;
+// Missing responses: 16-trait tiles, and fewer sample tiles per warp than the dense kernel so that the per-trait Gram band
+// buffers (32 KB) fit beside the X tile ring.
 template <int NT, bool CL>
 using CfgMis = SweepCfg<2, NT, CL, true>;
-template <int NT>
-bool pick_nt_mis(int nt, bool cl, int ncta, CfgInfo* out) {
-    if (nt == NT) {
-        if (!cl) *out = info<CfgMis<NT, false>>(1000 + NT, 1);
-        else if constexpr (NT <= kMaxNTMisCl) *out = info<CfgMis<NT, true>>(1100 + NT, ncta);
-        else return false;
-        return true;
-    }
-    if constexpr (NT < kMaxNTMis) return pick_nt_mis<NT + 1>(nt, cl, ncta, out);
-    return false;
-}
-// Which cluster size?  A cluster of c CTAs holds ceil(n / (112 c)) sample tiles per warp; smaller slices mean wider trait
-// tiles (more traits per serial chain step) but more CTAs to synchronise per block and fewer clusters per GPU.  Model,
-// fitted to sweeps timed on B200 (gpurun_out/r2_*.log: n = 1500 / 3000 / 5000, 2..8 CTAs):
-//   cycles per 8-SNP block  =  256 MT NT (tensor pipe: 4 warps per sub-partition x 4 MT NT DMMAs x 16 cycles)
-//                              + 1500 (S reduction -> chain -> -Delta hand-off across the cluster; + 500 for 8 CTAs)
-//   clusters resident at once on 148 SMs:  74 / 49 / 33 / 22 / 15  for  2 / 3 / 4 / 6 / 8 CTAs  (5 and 7 place badly)
-//   cost  =  rounds of the persistent grid x cycles per block  =  ceil(tiles / clusters) x ...
-// and the cheapest candidate wins: the choice depends on q_local through the number of rounds (C3 on one GPU, n = 3000,
-// q = 1500: 4 CTAs, 3 rounds of 16-trait tiles; C5 on 8 GPUs, n = 5000, q_local = 2500: 6 CTAs).
-int clusters_resident(int ncta, int sm_count) {
-    const int on148 = ncta == 1 ? 148 : ncta == 2 ? 74 : ncta == 3 ? 49 : ncta == 4 ? 33 : ncta == 6 ? 22 : 15;
-    return std::max(1, (int)((long)on148 * sm_count / 148));
-}
-template <class Pick>
-bool pick_by_cost(int n, int q, int sm_count, int max_nt_single, int max_nt_cl, int (*mt_of)(int, bool), Pick pick, CfgInfo* out) {
-    const char* fc = std::getenv("AQ_FORCE_CLUSTER");
-    const int forced = fc ? std::atoi(fc) : 0;
-    double best = 0.0;
-    int best_c = 0;
-    for (int c : {1, 2, 3, 4, 6, 8}) {
-        if (forced >= 1 && forced <= kMaxCluster && c != forced) continue;
-        const int nt = (n + 112 * c - 1) / (112 * c);
-        if (nt > (c == 1 ? max_nt_single : max_nt_cl)) continue;
-        const int mt = mt_of(nt, c > 1);
-        const long tiles = (q + 8 * mt - 1) / (8 * mt);
-        const long rounds = (tiles + clusters_resident(c, sm_count) - 1) / clusters_resident(c, sm_count);
-        const double cost = (double)rounds * (256.0 * mt * nt + (c == 1 ? 600.0 : 1500.0) + (c == 8 ? 500.0 : 0.0));
-        if (c == 1) { best_c = 1; break; }   // one CTA whenever the samples fit: no cluster traffic at all
-        if (!best_c || cost < best) { best = cost; best_c = c; }
-    }
-    if (forced >= 2 && forced <= kMaxCluster && !best_c) {   // a forced size outside the candidate list (5, 7)
-        const int nt = (n + 112 * forced - 1) / (112 * forced);
-        if (nt <= max_nt_cl) best_c = forced;
-    }
-    if (!best_c) return false;
-    const int nt = (n + 112 * best_c - 1) / (112 * best_c);
-    return pick(nt, best_c > 1, best_c, out);
-}
-int mt_dense(int nt, bool cl) { return mt_of_nt(nt, cl); }
-int mt_mis(int, bool) { return 2; }
+// One compiled configuration (an entry of kSweepKernels).
+struct SweepKernel {
+    bool mis, cl;                     // missing-response variant; sample-split cluster variant
+    int nt, n_pad, xs, kT, threads;   // n_pad: samples per CTA (slice), padded
+    size_t smem, tile_doubles;
+    int (*launch)(aq_ctx*, const SweepParams&);   // one sweep (mode 0) or residual set-up (mode 1) of a context
+};
+// the configuration a context runs: an entry of kSweepKernels and its number of CTAs per cluster (sample slices)
+struct CfgInfo {
+    const SweepKernel* k = nullptr;
+    int ncta = 1;
+};
 
-bool pick_cfg_mis(int n, int q, int sm_count, CfgInfo* out) {
-    return pick_by_cost(n, q, sm_count, kMaxNTMis, kMaxNTMisCl, mt_mis, pick_nt_mis<1>, out);
-}
-
-// development knob for both: AQ_FORCE_CLUSTER=1..8 fixes the number of CTAs per cluster
-bool pick_cfg(int n, int q, int sm_count, CfgInfo* out) {
-    return pick_by_cost(n, q, sm_count, kMaxNT, kMaxNTCl, mt_dense, pick_nt<1>, out);
+// Test and development overrides, read from the environment once, when a context is created, so that no other thread's
+// setenv can change the plan of a context while it sweeps:
+//   AQ_NO_TAIL               (any value) leftover traits go through full-size tiles, never the 8-trait tail variant
+//   AQ_NO_SEG                (any value) the SNP blocks of a tile are never cut into segments
+//   AQ_NSEG=S                S segments per tile whenever the tiles outnumber one round of the persistent grid
+//   AQ_FORCE_CLUSTER=c       c CTAs per cluster (1..8) wherever the samples fit
+//   AQ_MIS_KERNEL=warp|tile  the kernel aq_set_missing chooses for missing responses
+struct DevOverrides {
+    bool no_tail = false, no_seg = false;
+    int nseg = 0, force_cluster = 0;      // 0: not forced
+    bool mis_warp = false, mis_tile = false;
+};
+DevOverrides read_overrides() {
+    DevOverrides o;
+    o.no_tail = std::getenv("AQ_NO_TAIL") != nullptr;
+    o.no_seg = std::getenv("AQ_NO_SEG") != nullptr;
+    if (const char* v = std::getenv("AQ_NSEG")) o.nseg = std::max(1, std::atoi(v));   // (< 2: no segment count matches)
+    if (const char* v = std::getenv("AQ_FORCE_CLUSTER")) o.force_cluster = std::atoi(v);
+    if (const char* v = std::getenv("AQ_MIS_KERNEL")) {
+        o.mis_warp = std::strcmp(v, "warp") == 0;
+        o.mis_tile = std::strcmp(v, "tile") == 0;
+    }
+    return o;
 }
 
 }  // namespace
@@ -146,6 +96,7 @@ struct aq_ctx {
     int device = 0, n = 0, p = 0, q = 0;
     int p_pad = 0, q_pad = 0, nb = 0, ntiles = 0, sm_count = 0, ld_resid = 0;
     CfgInfo cfg{};
+    DevOverrides ov;
     cudaStream_t stream = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;  // sweep kernel
     cudaEvent_t evr0 = nullptr, evr1 = nullptr, evt0 = nullptr, evt1 = nullptr;  // rowsums / tables kernels
@@ -215,6 +166,32 @@ namespace {
 
 int build_gk(aq_ctx* c);   // (missing-response tile path, defined with aq_set_missing)
 
+// Launch configuration of kernel configuration C on the context's stream: clusters of cfg.ncta CTAs for the clustered
+// variant and, with `cooperative`, all CTAs resident at the same time.  lc.attrs points into `attr`.
+template <class C>
+cudaLaunchConfig_t launch_config(const aq_ctx* c, unsigned grid, bool cooperative, cudaLaunchAttribute (&attr)[2]) {
+    cudaLaunchConfig_t lc{};
+    lc.gridDim = dim3(grid);
+    lc.blockDim = dim3(C::kThreads);
+    lc.dynamicSmemBytes = C::kSmemBytes;
+    lc.stream = c->stream;
+    lc.attrs = attr;
+    lc.numAttrs = 0;
+    if (C::kCl) {
+        attr[lc.numAttrs].id = cudaLaunchAttributeClusterDimension;
+        attr[lc.numAttrs].val.clusterDim.x = c->cfg.ncta;
+        attr[lc.numAttrs].val.clusterDim.y = 1;
+        attr[lc.numAttrs].val.clusterDim.z = 1;
+        lc.numAttrs++;
+    }
+    if (cooperative) {
+        attr[lc.numAttrs].id = cudaLaunchAttributeCooperative;
+        attr[lc.numAttrs].val.cooperative = 1;
+        lc.numAttrs++;
+    }
+    return lc;
+}
+
 // Launch attributes of one kernel configuration on this context's device: set once per context (not in function statics:
 // the cluster size is a run-time value of the same template instance, and contexts live on several devices / threads).
 template <class C>
@@ -224,18 +201,8 @@ int prepare_sweep_t(aq_ctx* c, int slot) {
     AQ_CUDA(cudaFuncSetAttribute(sweep_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::kSmemBytes));
     c->max_groups[slot] = c->sm_count;
     if (C::kCl) {
-        cudaLaunchConfig_t lc{};
-        lc.blockDim = dim3(C::kThreads);
-        lc.dynamicSmemBytes = C::kSmemBytes;
-        lc.stream = c->stream;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = ncta;
-        attr[0].val.clusterDim.y = 1;
-        attr[0].val.clusterDim.z = 1;
-        lc.attrs = attr;
-        lc.numAttrs = 1;
-        lc.gridDim = dim3(c->sm_count / ncta * ncta);
+        cudaLaunchAttribute attr[2];
+        const cudaLaunchConfig_t lc = launch_config<C>(c, c->sm_count / ncta * ncta, false, attr);
         int nc = 0;
         AQ_CUDA(cudaOccupancyMaxActiveClusters(&nc, sweep_kernel<C>, &lc));
         if (nc < 1) return fail(AQ_EUNSUPPORTED, "no thread-block cluster of the required size can be scheduled");
@@ -256,31 +223,13 @@ int launch_sweep_t(aq_ctx* c, int slot, SweepParams P, int ntiles, int k_base) {
     int rc = prepare_sweep_t<C>(c, slot);
     if (rc != AQ_OK) return rc;
     if (ntiles <= 0) return AQ_OK;
-    const int ncta = c->cfg.ncta;
-    cudaLaunchConfig_t lc{};
-    lc.blockDim = dim3(C::kThreads);
-    lc.dynamicSmemBytes = C::kSmemBytes;
-    lc.stream = c->stream;
-    cudaLaunchAttribute attr[2];
-    lc.attrs = attr;
-    lc.numAttrs = 0;
-    if (C::kCl) {
-        attr[lc.numAttrs].id = cudaLaunchAttributeClusterDimension;
-        attr[lc.numAttrs].val.clusterDim.x = ncta;
-        attr[lc.numAttrs].val.clusterDim.y = 1;
-        attr[lc.numAttrs].val.clusterDim.z = 1;
-        lc.numAttrs++;
-    }
-    if (P.nseg > 1) {
-        // CTAs hand trait tiles over to one another inside the launch: all of them must be resident at the same time
-        attr[lc.numAttrs].id = cudaLaunchAttributeCooperative;
-        attr[lc.numAttrs].val.cooperative = 1;
-        lc.numAttrs++;
-    }
     P.ntiles = ntiles;
     P.k_base = k_base;
     const long nunits = (long)ntiles * P.nseg;
-    lc.gridDim = dim3((unsigned)std::min<long>(nunits, c->max_groups[slot]) * ncta);
+    // (segmented: CTAs hand trait tiles over to one another inside the launch, so all of them must be resident at once)
+    cudaLaunchAttribute attr[2];
+    const cudaLaunchConfig_t lc =
+        launch_config<C>(c, (unsigned)std::min<long>(nunits, c->max_groups[slot]) * c->cfg.ncta, P.nseg > 1, attr);
     AQ_CUDA(cudaLaunchKernelEx(&lc, sweep_kernel<C>, P));
     AQ_CUDA(cudaGetLastError());
     c->launches++;
@@ -300,14 +249,14 @@ struct SweepPlan {
 };
 constexpr double kSegOverheadBlocks = 4.0, kTailTileCost = 0.68;
 
-SweepPlan plan_sweep(const aq_ctx* c, int G, int kT, bool clustered, bool has_tail_variant) {
+SweepPlan plan_sweep(const aq_ctx* c, int G, int kT, bool has_tail_variant) {
     SweepPlan pl;
     const int ntiles = c->ntiles, nb = c->nb;
     pl.n_main = ntiles;
     pl.seg_len = nb;
     const int rem = ntiles % G;
     double best = (double)((ntiles + G - 1) / G) * (nb + kSegOverheadBlocks);
-    if (has_tail_variant && rem != 0 && !std::getenv("AQ_NO_TAIL")) {
+    if (has_tail_variant && rem != 0 && !c->ov.no_tail) {
         const int k_tail = (ntiles - rem) * kT;
         const int tail_tiles = (c->q - k_tail + 7) / 8;
         if (tail_tiles <= G) {
@@ -320,15 +269,15 @@ SweepPlan plan_sweep(const aq_ctx* c, int G, int kT, bool clustered, bool has_ta
             }
         }
     }
-    if (ntiles > G && !std::getenv("AQ_NO_SEG") && !(clustered && std::getenv("AQ_NO_SEG_CLUSTER"))) {
-        const char* force = std::getenv("AQ_NSEG");
+    if (ntiles > G && !c->ov.no_seg) {
+        const int force = c->ov.nseg;
         for (int S = 2; S <= 64 && nb / S >= 16; ++S) {
-            if (force && S != std::atoi(force)) continue;
+            if (force && S != force) continue;
             const int len = (nb + S - 1) / S;
             const int S2 = (nb + len - 1) / len;   // segments actually needed at this length
             const long slots = std::max<long>(S2, ((long)ntiles * S2 + G - 1) / G);
             const double cost = (double)slots * (len + kSegOverheadBlocks);
-            if (cost < best * 0.995 || (force && S == std::atoi(force))) {
+            if (cost < best * 0.995 || force) {
                 best = cost;
                 pl = SweepPlan{};
                 pl.nseg = S2;
@@ -348,7 +297,7 @@ int launch_sweep_cfg(aq_ctx* c, const SweepParams& P) {
     if (rc != AQ_OK) return rc;
     const int G = c->max_groups[0];
     const int ntiles = c->ntiles;
-    const SweepPlan pl = plan_sweep(c, G, Main::kT, CL, Main::MT > 1);
+    const SweepPlan pl = plan_sweep(c, G, Main::kT, Main::MT > 1);
     SweepParams Pm = P, Pt = P;
     Pm.nseg = pl.nseg;
     Pm.seg_len = pl.seg_len;
@@ -374,7 +323,7 @@ int launch_sweep_cfg(aq_ctx* c, const SweepParams& P) {
         // (measured: +0.5-1 % on a tensor-bound tile, +2.5 % on the chain-bound 8-trait tail tiles and cluster tiles, whose
         // helper warp sits closer to the serial path; the streaming pass costs 24 B per update, i.e. 2-6 % of a sweep for
         // n <= 1008 and < 1 % beyond.  So: full-size single-CTA tiles only; the tail's traits get one streamed extra row.)
-        if (c->rowpart && pl.n_main > 0 && pl.n_main + 1 <= c->rowpart_cap && !std::getenv("AQ_NO_ROWPART")) {
+        if (c->rowpart && pl.n_main > 0 && pl.n_main + 1 <= c->rowpart_cap) {
             Pm.rowpart = c->rowpart;
             Pm.rowpart_base = 0;
             c->rowpart_rows = pl.n_main;
@@ -407,29 +356,75 @@ int launch_sweep_mis_cfg(aq_ctx* c, const SweepParams& P) {
     return AQ_OK;
 }
 
-template <int NT>
-int launch_sweep_mis_id(aq_ctx* c, const SweepParams& P) {
-    if (c->cfg.id == 1000 + NT) return launch_sweep_mis_cfg<NT, false>(c, P);
-    if constexpr (NT <= kMaxNTMisCl)
-        if (c->cfg.id == 1100 + NT) return launch_sweep_mis_cfg<NT, true>(c, P);
-    if constexpr (NT < kMaxNTMis) return launch_sweep_mis_id<NT + 1>(c, P);
-    return fail(AQ_EUNSUPPORTED, "no kernel configuration (missing responses)");
+// ---- the compiled configurations.  A dense entry launches SweepCfg<1, NT, CL> as its 8-trait tail variant.
+template <class C>
+constexpr SweepKernel entry(int (*launch)(aq_ctx*, const SweepParams&)) {
+    return SweepKernel{C::kMis, C::kCl, C::NT, C::kNPad, C::kXS, C::kT, C::kThreads, C::kSmemBytes, C::kTileDoubles, launch};
+}
+template <int NT, bool CL>
+constexpr SweepKernel dense() { return entry<CfgOf<NT, CL>>(launch_sweep_cfg<NT, CL>); }
+template <int NT, bool CL>
+constexpr SweepKernel mis() { return entry<CfgMis<NT, CL>>(launch_sweep_mis_cfg<NT, CL>); }
+constexpr SweepKernel kSweepKernels[] = {
+    // dense, one CTA: NT 1-9 (n <= 1008)
+    dense<1, false>(), dense<2, false>(), dense<3, false>(), dense<4, false>(), dense<5, false>(), dense<6, false>(),
+    dense<7, false>(), dense<8, false>(), dense<9, false>(),
+    // dense, clustered: NT 1-8 (the leader also buffers the followers' S tiles: n <= ncta * 896)
+    dense<1, true>(), dense<2, true>(), dense<3, true>(), dense<4, true>(), dense<5, true>(), dense<6, true>(),
+    dense<7, true>(), dense<8, true>(),
+    // missing responses, one CTA: NT 1-7 (n <= 784)
+    mis<1, false>(), mis<2, false>(), mis<3, false>(), mis<4, false>(), mis<5, false>(), mis<6, false>(), mis<7, false>(),
+    // missing responses, clustered: NT 1-6 (n <= ncta * 672)
+    mis<1, true>(), mis<2, true>(), mis<3, true>(), mis<4, true>(), mis<5, true>(), mis<6, true>(),
+};
+
+const SweepKernel* find_kernel(bool missing, bool cl, int nt) {
+    for (const SweepKernel& k : kSweepKernels)
+        if (k.mis == missing && k.cl == cl && k.nt == nt) return &k;
+    return nullptr;
 }
 
-template <int NT>
-int launch_sweep_id(aq_ctx* c, const SweepParams& P) {
-    if (c->cfg.id == NT) return launch_sweep_cfg<NT, false>(c, P);
-    if constexpr (NT <= kMaxNTCl)
-        if (c->cfg.id == 100 + NT) return launch_sweep_cfg<NT, true>(c, P);
-    if constexpr (NT < kMaxNT) return launch_sweep_id<NT + 1>(c, P);
-    return fail(AQ_EUNSUPPORTED, "no kernel configuration");
+// Which cluster size?  A cluster of c CTAs holds ceil(n / (112 c)) sample tiles per warp; smaller slices mean wider trait
+// tiles (more traits per serial chain step) but more CTAs to synchronise per block and fewer clusters per GPU.  Model,
+// fitted to sweeps timed on B200 (gpurun_out/r2_*.log: n = 1500 / 3000 / 5000, 2..8 CTAs):
+//   cycles per 8-SNP block  =  256 MT NT (tensor pipe: 4 warps per sub-partition x 4 MT NT DMMAs x 16 cycles)
+//                              + 1500 (S reduction -> chain -> -Delta hand-off across the cluster; + 500 for 8 CTAs)
+//   clusters resident at once on 148 SMs:  74 / 49 / 33 / 22 / 15  for  2 / 3 / 4 / 6 / 8 CTAs  (5 and 7 place badly)
+//   cost  =  rounds of the persistent grid x cycles per block  =  ceil(tiles / clusters) x ...
+// and the cheapest candidate wins: the choice depends on q_local through the number of rounds (C3 on one GPU, n = 3000,
+// q = 1500: 4 CTAs, 3 rounds of 16-trait tiles; C5 on 8 GPUs, n = 5000, q_local = 2500: 6 CTAs).
+int clusters_resident(int ncta, int sm_count) {
+    const int on148 = ncta == 1 ? 148 : ncta == 2 ? 74 : ncta == 3 ? 49 : ncta == 4 ? 33 : ncta == 6 ? 22 : 15;
+    return std::max(1, (int)((long)on148 * sm_count / 148));
+}
+// The dense or missing-response configuration for n samples and q traits; `forced` (1..8) fixes the cluster size.  No
+// entry (k == NULL) when n is beyond every configuration of the kind.
+CfgInfo pick_cfg(int n, int q, int sm_count, bool missing, int forced) {
+    double best = 0.0;
+    CfgInfo pick;
+    for (int c : {1, 2, 3, 4, 6, 8}) {
+        if (forced >= 1 && forced <= kMaxCluster && c != forced) continue;
+        const SweepKernel* k = find_kernel(missing, c > 1, (n + 112 * c - 1) / (112 * c));
+        if (!k) continue;
+        const int mt = k->kT / 8, nt = k->nt;
+        const long tiles = (q + 8 * mt - 1) / (8 * mt);
+        const long rounds = (tiles + clusters_resident(c, sm_count) - 1) / clusters_resident(c, sm_count);
+        const double cost = (double)rounds * (256.0 * mt * nt + (c == 1 ? 600.0 : 1500.0) + (c == 8 ? 500.0 : 0.0));
+        if (c == 1) { pick = CfgInfo{k, 1}; break; }   // one CTA whenever the samples fit: no cluster traffic at all
+        if (!pick.k || cost < best) { best = cost; pick = CfgInfo{k, c}; }
+    }
+    if (forced >= 2 && forced <= kMaxCluster && !pick.k) {   // a forced size outside the candidate list (5, 7)
+        const SweepKernel* k = find_kernel(missing, true, (n + 112 * forced - 1) / (112 * forced));
+        if (k) pick = CfgInfo{k, forced};
+    }
+    return pick;
 }
 
 int launch_sweep(aq_ctx* c, int mode, double cc, double log_sig2_inv) {
     SweepParams P;
     P.order = c->order_dev;
     P.xtiles = c->xtiles;
-    P.tile_stride = c->cfg.tile_doubles;
+    P.tile_stride = c->cfg.k->tile_doubles;
     P.nb = c->nb;
     P.ntiles = c->ntiles;
     P.k_base = 0;
@@ -480,8 +475,7 @@ int launch_sweep(aq_ctx* c, int mode, double cc, double log_sig2_inv) {
         P.timing = tbuf;
     }
 #endif
-    if (c->cfg.id >= 1000) return launch_sweep_mis_id<1>(c, P);
-    return launch_sweep_id<1>(c, P);
+    return c->cfg.k->launch(c, P);
 }
 
 int upload_pxq(aq_ctx* c, const double* host, double* dev) {
@@ -531,10 +525,10 @@ int retile(aq_ctx* c) {
     c->order_pad.assign(c->p_pad, -1);  // padding slots of the last block carry -1, as in the tile images
     std::copy(c->order.begin(), c->order.end(), c->order_pad.begin());
     AQ_CUDA(cudaMemcpyAsync(c->order_dev, c->order_pad.data(), sizeof(int32_t) * c->p_pad, cudaMemcpyHostToDevice, c->stream));
-    build_tiles_kernel<<<dim3(c->nb, c->cfg.ncta), 256, 0, c->stream>>>(c->xraw, c->order_dev, c->n, c->p, c->cfg.xs,
-                                                                         c->cfg.n_pad, c->cfg.tile_doubles, c->xtiles);
+    build_tiles_kernel<<<dim3(c->nb, c->cfg.ncta), 256, 0, c->stream>>>(c->xraw, c->order_dev, c->n, c->p, c->cfg.k->xs,
+                                                                         c->cfg.k->n_pad, c->cfg.k->tile_doubles, c->xtiles);
     AQ_CUDA(cudaGetLastError());
-    gram_band_kernel<<<c->nb, 128, 0, c->stream>>>(c->xtiles, c->cfg.n_pad, c->cfg.ncta, c->cfg.xs, c->cfg.tile_doubles);
+    gram_band_kernel<<<c->nb, 128, 0, c->stream>>>(c->xtiles, c->cfg.k->n_pad, c->cfg.ncta, c->cfg.k->xs, c->cfg.k->tile_doubles);
     AQ_CUDA(cudaGetLastError());
     c->launches += 2;
     return AQ_OK;
@@ -647,8 +641,9 @@ int create_impl(aq_ctx** out, int device, int n, int p, int q_local, const doubl
     int sm = 0;
     int rc = aq_device_info(device, &sm, nullptr, nullptr);
     if (rc != AQ_OK) return rc;
-    CfgInfo cfg;
-    if (!pick_cfg(n, q_local, sm, &cfg))
+    const DevOverrides ov = read_overrides();
+    const CfgInfo cfg = pick_cfg(n, q_local, sm, false, ov.force_cluster);
+    if (!cfg.k)
         return fail(AQ_EUNSUPPORTED, "aq_create: n > 7168 is beyond the 8-CTA sample-split cluster kernel");
     aq_ctx* c = new aq_ctx();
     c->device = device;
@@ -656,14 +651,15 @@ int create_impl(aq_ctx** out, int device, int n, int p, int q_local, const doubl
     c->p = p;
     c->q = q_local;
     c->cfg = cfg;
+    c->ov = ov;
     c->sm_count = sm;
     c->p_pad = (p + kBlk - 1) / kBlk * kBlk;
     // leading dimension of the p x q arrays: a multiple of every tile width (16 / 24 / 32 traits, 96 = their lcm), so that a
     // context can change its kernel configuration (missing responses use 16-trait tiles) without re-laying them out
     c->q_pad = (q_local + 95) / 96 * 96;
     c->nb = c->p_pad / kBlk;
-    c->ld_resid = cfg.n_pad * cfg.ncta;
-    c->ntiles = (q_local + cfg.kT - 1) / cfg.kT;
+    c->ld_resid = cfg.k->n_pad * cfg.ncta;
+    c->ntiles = (q_local + cfg.k->kT - 1) / cfg.k->kT;
     const size_t pq = (size_t)c->p_pad * c->q_pad;
     c->stage_cols = (int)std::max<size_t>(1, std::min<size_t>((size_t)q_local, ((size_t)256 << 20) / (sizeof(double) * (size_t)p)));
     c->n_partials = (size_t)((c->q + 255) / 256) * ((c->p + kTabRowsPerBlock - 1) / kTabRowsPerBlock);
@@ -677,7 +673,7 @@ int create_impl(aq_ctx** out, int device, int n, int p, int q_local, const doubl
         }                                                                                 \
     } while (0)
     AQ_ALLOC(c->xraw, (size_t)n * p);
-    AQ_ALLOC(c->xtiles, (size_t)c->nb * cfg.ncta * cfg.tile_doubles);
+    AQ_ALLOC(c->xtiles, (size_t)c->nb * cfg.ncta * cfg.k->tile_doubles);
     AQ_ALLOC(c->ymat, (size_t)c->q_pad * c->ld_resid);
     AQ_ALLOC(c->resid, (size_t)c->q_pad * c->ld_resid);
     AQ_ALLOC(c->gam, pq);
@@ -1266,8 +1262,8 @@ namespace {
 int build_gk(aq_ctx* c) {
     const int ntiles = c->ntiles;
     AQ_CUDA(cudaMemsetAsync(c->xnsq, 0, sizeof(double) * (size_t)c->p_pad * c->q_pad, c->stream));
-    gk_build_kernel<<<dim3(c->nb, ntiles), 128, 0, c->stream>>>(c->xtiles, c->nb, c->cfg.ncta, c->cfg.n_pad, c->cfg.xs,
-                                                                c->cfg.tile_doubles, c->mis_off_dev, c->mis_idx_dev, c->q,
+    gk_build_kernel<<<dim3(c->nb, ntiles), 128, 0, c->stream>>>(c->xtiles, c->nb, c->cfg.ncta, c->cfg.k->n_pad, c->cfg.k->xs,
+                                                                c->cfg.k->tile_doubles, c->mis_off_dev, c->mis_idx_dev, c->q,
                                                                 c->q_pad, c->gk, c->xnsq);
     AQ_CUDA(cudaGetLastError());
     c->launches++;
@@ -1280,8 +1276,8 @@ int build_gk(aq_ctx* c) {
 int set_missing_tile(aq_ctx* c, const CfgInfo& cfgm, const double* mis_pat, double* n_obs) {
     const size_t pq = (size_t)c->p_pad * c->q_pad;
     const int n = c->n, q = c->q;
-    if (cfgm.id != c->cfg.id || cfgm.ncta != c->cfg.ncta) {
-        const int ld_new = cfgm.n_pad * cfgm.ncta;
+    if (cfgm.k != c->cfg.k || cfgm.ncta != c->cfg.ncta) {
+        const int ld_new = cfgm.k->n_pad * cfgm.ncta;
         double *y_new = nullptr, *r_new = nullptr, *t_new = nullptr;
         AQ_CUDA(cudaStreamSynchronize(c->stream));
         AQ_CUDA(cudaFree(c->xtiles));
@@ -1297,11 +1293,11 @@ int set_missing_tile(aq_ctx* c, const CfgInfo& cfgm, const double* mis_pat, doub
         c->ymat = y_new;
         AQ_CUDA(cudaMalloc((void**)&r_new, sizeof(double) * (size_t)c->q_pad * ld_new));
         c->resid = r_new;
-        AQ_CUDA(cudaMalloc((void**)&t_new, sizeof(double) * (size_t)c->nb * cfgm.ncta * cfgm.tile_doubles));
+        AQ_CUDA(cudaMalloc((void**)&t_new, sizeof(double) * (size_t)c->nb * cfgm.ncta * cfgm.k->tile_doubles));
         c->xtiles = t_new;
         c->cfg = cfgm;
         c->ld_resid = ld_new;
-        c->ntiles = (q + cfgm.kT - 1) / cfgm.kT;
+        c->ntiles = (q + cfgm.k->kT - 1) / cfgm.k->kT;
         c->attr_done[0] = c->attr_done[1] = false;
         if (c->seg_done) { cudaFree(c->seg_done); c->seg_done = nullptr; }
         if (c->rowpart) { cudaFree(c->rowpart); c->rowpart = nullptr; }
@@ -1367,22 +1363,20 @@ int aq_set_missing(aq_ctx* c, const double* mis_pat, double* n_obs) {
     // Two kernels serve coreDualMisLoop: the tile-structured one (the blocked tensor-core sweep with masked accumulators
     // and a per-trait Gram band table of 128 B per SNP x trait pair, n <= 5376) and the warp-per-trait one (no table,
     // n <= 2048, ~8x slower).  The tile path is taken whenever its table fits beside the rest; AQ_MIS_KERNEL=warp|tile forces.
-    const char* force = std::getenv("AQ_MIS_KERNEL");
-    const bool want_warp = force && std::strcmp(force, "warp") == 0, want_tile = force && std::strcmp(force, "tile") == 0;
-    CfgInfo cfgm;
-    bool tile_ok = !want_warp && pick_cfg_mis(c->n, c->q, c->sm_count, &cfgm);
+    const CfgInfo cfgm = c->ov.mis_warp ? CfgInfo{} : pick_cfg(c->n, c->q, c->sm_count, true, c->ov.force_cluster);
+    bool tile_ok = cfgm.k != nullptr;
     if (tile_ok) {
         size_t fr = 0, tot = 0;
         AQ_CUDA(cudaMemGetInfo(&fr, &tot));
         const size_t ntiles16 = (size_t)(c->q + 15) / 16;
         const double need = 8.0 * (double)ntiles16 * c->nb * 128 * 16 + 3.0 * 8.0 * (double)pq +
-                            8.0 * (double)c->nb * cfgm.ncta * (double)cfgm.tile_doubles +
-                            16.0 * (double)c->q_pad * cfgm.n_pad * cfgm.ncta + (double)((size_t)256 << 20);
-        const double freed = 8.0 * (double)c->nb * c->cfg.ncta * (double)c->cfg.tile_doubles + 16.0 * (double)c->q_pad * c->ld_resid;
+                            8.0 * (double)c->nb * cfgm.ncta * (double)cfgm.k->tile_doubles +
+                            16.0 * (double)c->q_pad * cfgm.k->n_pad * cfgm.ncta + (double)((size_t)256 << 20);
+        const double freed = 8.0 * (double)c->nb * c->cfg.ncta * (double)c->cfg.k->tile_doubles + 16.0 * (double)c->q_pad * c->ld_resid;
         if (need > (double)fr + freed) tile_ok = false;
     }
     if (tile_ok) return set_missing_tile(c, cfgm, mis_pat, n_obs);
-    if (want_tile) return fail(AQ_EUNSUPPORTED, "aq_set_missing: the tile-structured kernel needs n <= 5376 and 128 B per SNP x trait pair");
+    if (c->ov.mis_tile) return fail(AQ_EUNSUPPORTED, "aq_set_missing: the tile-structured kernel needs n <= 5376 and 128 B per SNP x trait pair");
     if (c->n > 2048)
         return fail(AQ_EUNSUPPORTED, "aq_set_missing: no room for the tile kernel's Gram band table (128 B per SNP x trait pair) "
                                      "and the warp-per-trait kernel covers n <= 2048 only");
@@ -1544,7 +1538,7 @@ int64_t aq_launch_count(const aq_ctx* c) { return c ? c->launches : 0; }
 
 int aq_sweep_plan(const aq_ctx* c, int* traits_per_tile, int* ntiles, int* groups, int* nseg) {
     if (!c) return fail(AQ_EINVAL, "NULL context");
-    if (traits_per_tile) *traits_per_tile = c->cfg.kT;
+    if (traits_per_tile) *traits_per_tile = c->cfg.k->kT;
     if (ntiles) *ntiles = c->ntiles;
     if (groups) *groups = c->max_groups[0];
     if (nseg) *nseg = c->last_nseg;

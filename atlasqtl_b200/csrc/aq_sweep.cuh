@@ -37,16 +37,6 @@
 #define AQ_T0() do { } while (0)
 #endif
 
-// Where the pending S phase is finished (accumulator chains added, partials stored, chain warp told) relative to the rank-8
-// update of the previous block: -1 = before the update starts (default); 0 / 2 / ... = after that many sample tiles of the
-// update, so that the S accumulators drain behind the first update DMMAs instead of idling the tensor pipe at the phase
-// boundary.  Measured on B200 (n = 1000, p = 50000, 2500 traits, gpurun_out/r2d.log): -1: 18.63 ms, 0: 19.01 ms, 2: 19.43 ms
-// -- the later the S partials reach the chain warp, the slower the sweep, although the chain warp idles 40 % of a block:
-// kept as a build-time knob for the record, off by default.
-#ifndef AQ_S_FINISH_AT
-#define AQ_S_FINISH_AT -1
-#endif
-
 namespace aq {
 
 struct SweepParams {
@@ -120,9 +110,6 @@ struct SweepCfg {
     // the chain's logistic with two dependent operations less (aq_common.cuh): wins where the serial chain bounds a block
     // (clusters, missing responses, 24- / 32-trait tiles of small n), loses on the tensor-bound 16-trait tiles
     static constexpr bool kShortLogistic = CL_ || MIS_ || MT_ != 2;
-    // where the pending S phase is finished inside the rank-8 update (see AQ_S_FINISH_AT); with 3 or 4 M tiles per warp the
-    // S accumulators kept alive across the phase boundary would cost register spills in the MMA loops: never pipelined there
-    static constexpr int kSFin = (MT_ <= 2) ? AQ_S_FINISH_AT : -1;
     static constexpr size_t kTileDoubles = (size_t)kBlk * kXS + kTileTail;
     // S tiles in shared memory ([trait][8 SNP slots], partials and sums alike): row stride 8 doubles, the four 16-byte
     // pairs of a row XOR-swizzled by (trait >> 1) & 3 (sp_off), so that both the C-fragment stores of the MMA warps (lanes
@@ -130,44 +117,56 @@ struct SweepCfg {
     // pair) hit 8 different 16-byte bank groups.  (ncu on the unswizzled stride-10 layout: 2-way conflicts on every
     // partial store, 15 % of the kernel's shared-memory wavefronts.)
     static constexpr int kSps = 8;
-    static constexpr size_t kSpartDoubles = (size_t)WS * kT * kSps;      // [WS][kT][kSps], single-buffered (sfree barrier)
     // who sums the split-K partials of S: the chain warp itself (single CTA: one hop less between the tensor work and the
     // recurrence), or the helper warp (clusters: the wait for the other CTAs' slices stays off the serial path)
     static constexpr bool kChainSums = MT > 1;
     // cluster leader: the helper warp sums the other CTAs' S tiles while the chain warp sums this CTA's own partials
     // (n = 5000, 8 CTAs: chain does both 24.99 ms, in parallel 23.74 ms; helper does both, as in round 1: 28.4 ms)
     static constexpr bool kHelperSumsFollowers = kCl && kChainSums;
-    // who forwards -Delta to the other CTAs of a cluster in sweep mode: the leader's MMA warps when they start the update
-    // (448 threads, ~2 stores each) -- or the chain warp itself, straight from its registers, before it publishes locally
-    // (28 stores per lane, but the followers' copy leaves a barrier wake-up and a shared-memory round trip earlier).  The
-    // helper warp doing it after the publish was far slower (n = 5000: 23.7 -> 34.8 ms, gpurun_out/r2_ab4.log).
-#ifdef AQ_AB_CHAIN_FWD
-    static constexpr bool kChainForwards = kCl && kChainSums;
-#else
-    static constexpr bool kChainForwards = false;
-#endif
+    static constexpr int kIoPer = kMis ? 4 : 2;        // iobuf entries per (SNP slot, trait)
+    static constexpr int kStgArrays = kMis ? 8 : 5;    // p x q arrays staged per block
+    static constexpr uint32_t kDeltaBytes = (uint32_t)(kT * kBlk * sizeof(double));  // one -Delta block (or S tile)
+
+    // ---- shared-memory layout: offset and size (doubles) of every region, each starting where the previous one ends (size 0
+    // where a configuration has no use for it), then the barrier block.  The kernel carves its pointers from these.
+    // [kStages] X tile images: the ring the producer lane fills with bulk copies
+    static constexpr size_t kOffTiles = 0, kTilesDoubles = kStages * kTileDoubles;
+    // [WS][kT][kSps] split-K partials of S, single-buffered (sfree barrier)
+    static constexpr size_t kOffSpart = kOffTiles + kTilesDoubles, kSpartDoubles = (size_t)WS * kT * kSps;
     // [2][kT][kSps] S tile handed from the helper to the chain: the whole sum (8-trait tiles) or the followers' part of it
-    static constexpr size_t kSsumDoubles = (kChainSums && !kHelperSumsFollowers) ? 0 : (size_t)2 * kT * kSps;
-    static constexpr size_t kDbufDoubles = (size_t)2 * kT * kBlk;
-    static constexpr size_t kRsqDoubles = (size_t)WS * kT;
+    static constexpr size_t kOffSsum = kOffSpart + kSpartDoubles,
+                            kSsumDoubles = (kChainSums && !kHelperSumsFollowers) ? 0 : (size_t)2 * kT * kSps;
+    // [2][kT x kBlk] -Delta (d_off layout)
+    static constexpr size_t kOffDbuf = kOffSsum + kSsumDoubles, kDbufDoubles = (size_t)2 * kT * kBlk;
+    // [WS][kT] squared norms of the residual, per MMA warp
+    static constexpr size_t kOffRsqs = kOffDbuf + kDbufDoubles, kRsqsDoubles = (size_t)WS * kT;
     // [2][kBlk][kIoPer][kT]: in beta_old, c (D + cst) (+ a, bq per pair with missing responses); out gam, mu
-    static constexpr int kIoPer = kMis ? 4 : 2;
-    static constexpr size_t kIoDoubles = (size_t)2 * kBlk * kIoPer * kT;
+    static constexpr size_t kOffIo = kOffRsqs + kRsqsDoubles, kIoDoubles = (size_t)2 * kBlk * kIoPer * kT;
     // [kStgArrays][kBlk][kT]: gam, mu, D, W, I0 (+ X_norm_sq, a, log sig2_beta) rows of the next block
-    static constexpr int kStgArrays = kMis ? 8 : 5;
-    static constexpr size_t kStgDoubles = (size_t)kStgArrays * kBlk * kT;
-    static constexpr size_t kGkDoubles = kMis ? (size_t)2 * 128 * kT : 0;   // [2][128][kT] per-trait Gram band of a block
-    static constexpr uint32_t kDeltaBytes = (uint32_t)(kT * kBlk * sizeof(double));  // one -Delta block
-    // cluster variant only: followers' reduced S tiles and squared-norm partials land in the leader's shared memory
-    static constexpr size_t kRedDoubles = kCl ? (size_t)2 * (kMaxCluster - 1) * kT * kSps : 0;
-    static constexpr size_t kRsqAllDoubles = kCl ? (size_t)(kMaxCluster - 1) * kT : 0;
-    // full, empty, dready, dcons, sred, rsqbar, inready, sfree, sdone [2][4]
-    static constexpr int kNumBars = 2 * kStages + 2 + 2 + 2 + 1 + 2 + 1 + 8;
-    static constexpr size_t kSmemBytes = (kStages * kTileDoubles + kSpartDoubles + kSsumDoubles + kDbufDoubles + kRsqDoubles +
-                                          kIoDoubles + kStgDoubles + kRedDoubles + kRsqAllDoubles + kGkDoubles) *
-                                             sizeof(double) +
-                                         24 * sizeof(uint64_t);
-    static_assert(kNumBars <= 24, "barrier block");
+    static constexpr size_t kOffStg = kOffIo + kIoDoubles, kStgDoubles = (size_t)kStgArrays * kBlk * kT;
+    // cluster leader: [2][kMaxCluster - 1][kT][kSps] the followers' reduced S tiles
+    static constexpr size_t kOffRed = kOffStg + kStgDoubles, kRedDoubles = kCl ? (size_t)2 * (kMaxCluster - 1) * kT * kSps : 0;
+    // cluster leader: [kMaxCluster - 1][kT] the followers' squared-norm partials
+    static constexpr size_t kOffRsqAll = kOffRed + kRedDoubles, kRsqAllDoubles = kCl ? (size_t)(kMaxCluster - 1) * kT : 0;
+    // missing responses: [2][128][kT] per-trait Gram band of a block
+    static constexpr size_t kOffGk = kOffRsqAll + kRsqAllDoubles, kGkDoubles = kMis ? (size_t)2 * 128 * kT : 0;
+    static constexpr size_t kOffBars = kOffGk + kGkDoubles;
+    // barrier block: slot of the first barrier of each family
+    static constexpr int kBarFull = 0;                      // [kStages] tile landed (tx bytes)
+    static constexpr int kBarEmpty = kBarFull + kStages;    // [kStages] MMA warps released the tile
+    static constexpr int kBarDready = kBarEmpty + kStages;  // [2] chain warp published -Delta (in every CTA of the cluster)
+    static constexpr int kBarDcons = kBarDready + 2;        // [2] mode 1 only, leader: all MMA warps consumed -Delta buffer
+    static constexpr int kBarSred = kBarDcons + 2;          // [2] leader: followers delivered their reduced S tiles
+    static constexpr int kBarRsq = kBarSred + 2;            // [1] leader: followers delivered their squared-norm partials
+    static constexpr int kBarInready = kBarRsq + 1;         // [2] helper warp staged S and the block's inputs for the chain
+    static constexpr int kBarSfree = kBarInready + 2;       // [1] helper / reducer warp has read the S partials of a block
+    // [2][4] this CTA's MMA warps wrote their S partials, one barrier per SM sub-partition (the four warps of SMSP 0, 1, 2,
+    // the two of SMSP 3): whoever sums the partials takes them group by group as they complete instead of after the last
+    static constexpr int kBarSdone = kBarSfree + 1;
+    static constexpr int kNumBars = kBarSdone + 8;
+    static constexpr int kBarSlots = 24;
+    static constexpr size_t kSmemBytes = kOffBars * sizeof(double) + kBarSlots * sizeof(uint64_t);
+    static_assert(kNumBars <= kBarSlots, "barrier block");
     static_assert(kT <= 32, "one chain lane per trait");
     static_assert(!kMis || kT == 16, "the missing-response variant uses 16-trait tiles (its Gram band table is laid out for them)");
     static_assert(kXS % 16 == 8, "row stride must be 8 mod 16 doubles");
@@ -241,21 +240,18 @@ __device__ __forceinline__ void sum_own_partials(double (&s)[kBlk], const double
     if (lane == 0) mbar_arrive(&sfree[0]);  // the MMA warps may overwrite the partials
 }
 
-// Cluster leader: the S tiles the other CTAs reduced and shipped here (st.async, accounted on sred).  Lane = trait; with
-// <= 16 traits per tile the two half-warps split the CTAs and the halves are added at the end.
+// Cluster leader: waits until the other CTAs' reduced S tiles of block gb have landed here (st.async, accounted on sred).
 template <class Cfg>
-__device__ __forceinline__ void sum_follower_tiles(double (&s)[kBlk], const double* red, uint64_t* sred, long gb, int ncta,
-                                                   int lane, int tsum) {
-    constexpr int kT = Cfg::kT;
-    constexpr int kH = (kT <= 16) ? 2 : 1;
-    const int half = (kH == 2) ? (lane >> 4) : 0;
-#pragma unroll
-    for (int t = 0; t < kBlk; ++t) s[t] = 0.0;
+__device__ __forceinline__ void wait_follower_tiles(uint64_t* sred, long gb, int ncta, int lane) {
     if (lane == 0) mbar_arrive_expect_tx(&sred[gb & 1], (uint32_t)(ncta - 1) * Cfg::kDeltaBytes);
     mbar_wait(&sred[gb & 1], (uint32_t)((gb >> 1) & 1));
-    const int mid = (kH == 2) ? (ncta + 1) / 2 : ncta;
-    for (int r2 = (half == 0 ? 1 : mid); r2 < (half == 0 ? mid : ncta); ++r2) {
-        const double* rp = red + (size_t)((gb & 1) * (kMaxCluster - 1) + (r2 - 1)) * kT * Cfg::kSps;
+}
+
+// Cluster leader: adds the S tiles of CTA ranks [r0, r1) to the row of trait `tsum`, in rank order.
+template <class Cfg>
+__device__ __forceinline__ void add_follower_tiles(double (&s)[kBlk], const double* red, long gb, int tsum, int r0, int r1) {
+    for (int r2 = r0; r2 < r1; ++r2) {
+        const double* rp = red + (size_t)((gb & 1) * (kMaxCluster - 1) + (r2 - 1)) * Cfg::kT * Cfg::kSps;
 #pragma unroll
         for (int t = 0; t < kBlk; t += 2) {
             const double2 v = *reinterpret_cast<const double2*>(rp + sp_off(tsum, t));
@@ -263,6 +259,20 @@ __device__ __forceinline__ void sum_follower_tiles(double (&s)[kBlk], const doub
             s[t + 1] += v.y;
         }
     }
+}
+
+// Cluster leader: the sum of the S tiles the other CTAs shipped here.  Lane = trait; with <= 16 traits per tile the two
+// half-warps split the CTAs and the halves are added at the end.
+template <class Cfg>
+__device__ __forceinline__ void sum_follower_tiles(double (&s)[kBlk], const double* red, uint64_t* sred, long gb, int ncta,
+                                                   int lane, int tsum) {
+    constexpr int kH = (Cfg::kT <= 16) ? 2 : 1;
+    const int half = (kH == 2) ? (lane >> 4) : 0;
+#pragma unroll
+    for (int t = 0; t < kBlk; ++t) s[t] = 0.0;
+    wait_follower_tiles<Cfg>(sred, gb, ncta, lane);
+    const int mid = (kH == 2) ? (ncta + 1) / 2 : ncta;
+    add_follower_tiles<Cfg>(s, red, gb, tsum, half == 0 ? 1 : mid, half == 0 ? mid : ncta);
     if (kH == 2) {
 #pragma unroll
         for (int t = 0; t < kBlk; ++t) s[t] += __shfl_xor_sync(0xffffffffu, s[t], 16);
@@ -279,19 +289,8 @@ __device__ __forceinline__ void sum_s_partials(double (&s)[kBlk], const double* 
     const int half = (kH == 2) ? (lane >> 4) : 0;
     sum_own_partials<Cfg>(s, spart, sdone, sfree, gb, lane, tsum);
     if (Cfg::kCl && ncta > 1) {  // + the other sample slices, already reduced (and stored here) by their CTAs
-        if (lane == 0) mbar_arrive_expect_tx(&sred[gb & 1], (uint32_t)(ncta - 1) * Cfg::kDeltaBytes);
-        mbar_wait(&sred[gb & 1], (uint32_t)((gb >> 1) & 1));
-        if (half == 0) {
-            for (int r2 = 1; r2 < ncta; ++r2) {
-                const double* rp = red + (size_t)((gb & 1) * (kMaxCluster - 1) + (r2 - 1)) * kT * Cfg::kSps;
-#pragma unroll
-                for (int t = 0; t < kBlk; t += 2) {
-                    const double2 v = *reinterpret_cast<const double2*>(rp + sp_off(tsum, t));
-                    s[t] += v.x;
-                    s[t + 1] += v.y;
-                }
-            }
-        }
+        wait_follower_tiles<Cfg>(sred, gb, ncta, lane);
+        if (half == 0) add_follower_tiles<Cfg>(s, red, gb, tsum, 1, ncta);
     }
     if (kH == 2) {
 #pragma unroll
@@ -351,29 +350,29 @@ __global__ void __launch_bounds__(Cfg::kThreads, 1) sweep_kernel(const SweepPara
     constexpr bool kCl = Cfg::kCl;
     constexpr bool kMis = Cfg::kMis;
     constexpr int kIoPer = Cfg::kIoPer;
+    // regions and barriers as SweepCfg lays them out
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    double* tiles = reinterpret_cast<double*>(smem_raw);
-    double* spart = tiles + kStages * Cfg::kTileDoubles;  // [WS][kT][kSps]
-    double* ssum = spart + Cfg::kSpartDoubles;            // [2][kT][kSps]  (clustered variant only)
-    double* dbuf = ssum + Cfg::kSsumDoubles;              // [2][kT x kBlk]  (holds -Delta, d_off layout)
-    double* rsqs = dbuf + Cfg::kDbufDoubles;              // [WS][kT]
-    double* iobuf = rsqs + Cfg::kRsqDoubles;              // [2][kBlk][2][kT]
-    double* stg = iobuf + Cfg::kIoDoubles;                // [5][kBlk][kT]
-    double* red = stg + Cfg::kStgDoubles;                 // leader: [2][kMaxCluster-1][kT][kSps]
-    double* rsq_all = red + Cfg::kRedDoubles;             // leader: [kMaxCluster-1][kT]
-    double* gkbuf = rsq_all + Cfg::kRsqAllDoubles;        // missing responses: [2][128][kT] per-trait Gram band
-    uint64_t* bars = reinterpret_cast<uint64_t*>(gkbuf + Cfg::kGkDoubles);
-    uint64_t* full = bars;                       // [kStages]  tile landed (tx bytes)
-    uint64_t* empty = bars + kStages;            // [kStages]  MMA warps released the tile
-    uint64_t* dready = bars + 2 * kStages;       // [2]  chain warp published -Delta (in every CTA of the cluster)
-    uint64_t* dcons = bars + 2 * kStages + 2;    // [2]  mode 1 only, leader: all MMA warps consumed -Delta buffer
-    uint64_t* sred = bars + 2 * kStages + 4;     // [2]  leader: followers delivered their reduced S tiles
-    uint64_t* rsqbar = bars + 2 * kStages + 6;   // [1]  leader: followers delivered their squared-norm partials
-    uint64_t* inready = bars + 2 * kStages + 7;  // [2]  helper warp staged S and the block's inputs for the chain
-    uint64_t* sfree = bars + 2 * kStages + 9;    // [1]  helper / reducer warp has read the S partials of a block
-    // [2][4]  this CTA's MMA warps wrote their S partials, one barrier per SM sub-partition (the four warps of SMSP 0, 1, 2,
-    // the two of SMSP 3): whoever sums the partials takes them group by group as they complete instead of after the last
-    uint64_t* sdone = bars + 2 * kStages + 10;
+    double* const smem = reinterpret_cast<double*>(smem_raw);
+    double* tiles = smem + Cfg::kOffTiles;
+    double* spart = smem + Cfg::kOffSpart;
+    double* ssum = smem + Cfg::kOffSsum;
+    double* dbuf = smem + Cfg::kOffDbuf;
+    double* rsqs = smem + Cfg::kOffRsqs;
+    double* iobuf = smem + Cfg::kOffIo;
+    double* stg = smem + Cfg::kOffStg;
+    double* red = smem + Cfg::kOffRed;
+    double* rsq_all = smem + Cfg::kOffRsqAll;
+    double* gkbuf = smem + Cfg::kOffGk;
+    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + Cfg::kOffBars);
+    uint64_t* full = bars + Cfg::kBarFull;
+    uint64_t* empty = bars + Cfg::kBarEmpty;
+    uint64_t* dready = bars + Cfg::kBarDready;
+    uint64_t* dcons = bars + Cfg::kBarDcons;
+    uint64_t* sred = bars + Cfg::kBarSred;
+    uint64_t* rsqbar = bars + Cfg::kBarRsq;
+    uint64_t* inready = bars + Cfg::kBarInready;
+    uint64_t* sfree = bars + Cfg::kBarSfree;
+    uint64_t* sdone = bars + Cfg::kBarSdone;
 
     const int wid = threadIdx.x >> 5, lane = threadIdx.x & 31;
 #ifdef AQ_TIMING
@@ -444,13 +443,12 @@ __global__ void __launch_bounds__(Cfg::kThreads, 1) sweep_kernel(const SweepPara
         const int g = lane >> 2, l = lane & 3;
         const int i0 = ws * NT * 8;                       // first sample of this warp inside the CTA's slice
         const int ig = rank * Cfg::kNPad + i0;            // ... and inside the residual row
-        constexpr int tr0 = 0;
         // lane-constant shared-memory offsets of the two operand patterns
         const int offS = g * XS + ((i0 + 2 * l) ^ ((g & 2) << 1));         // + nt*8   (16-byte loads)
         const int offU0 = l * XS + ((i0 + g) ^ ((l & 2) << 1));            // ks = 0, + nt*8
         const int offU1 = (l + 4) * XS + ((i0 + g) ^ ((l & 2) << 1));      // ks = 1 (snp l+4 has the same bit 1)
-        const int offD = d_off<kT>(tr0 + g, l);                            // -Delta[trait g][snp l]; + 16 mt, + 4 kT (snp l + 4)
-        const int offP = sp_off(tr0 + g, 2 * l);                           // S partial pair; + 64 mt
+        const int offD = d_off<kT>(g, l);                                  // -Delta[trait g][snp l]; + 16 mt, + 4 kT (snp l + 4)
+        const int offP = sp_off(g, 2 * l);                                 // S partial pair; + 64 mt
         uint32_t dcons_leader[2] = {0, 0}, rsqbar_leader = 0, rsq_all_leader = 0;
         if (kCl) {
             dcons_leader[0] = mapa_u32(&dcons[0], 0);
@@ -469,21 +467,18 @@ __global__ void __launch_bounds__(Cfg::kThreads, 1) sweep_kernel(const SweepPara
 #pragma unroll
                 for (int nt = 0; nt < NT; ++nt) {
                     const double2 v = __ldcg(reinterpret_cast<const double2*>(
-                        P.resid + (size_t)(k0 + tr0 + mt * 8 + g) * P.ld_resid + ig + nt * 8 + 2 * l));
+                        P.resid + (size_t)(k0 + mt * 8 + g) * P.ld_resid + ig + nt * 8 + 2 * l));
                     acc[mt][nt][0] = v.x;
                     acc[mt][nt][1] = v.y;
                 }
-            // S phase of block gbi, in two halves.  s_issue: the split-K DMMAs of S'^T = R^T X_b into the accumulators sa.
-            // s_finish: add the accumulator chains, store the partials, tell the chain warp (directly after s_issue unless
-            // the AQ_S_FINISH_AT experiment moves it into the rank-8 update of the previous block).
-            constexpr int kSC = (MT >= 4) ? 1 : 2;   // accumulator chains per M tile
+            constexpr int kSC = (MT >= 4) ? 1 : 2;   // accumulator chains per M tile of the S phase
             double sa[MT][2][2];
             // missing responses: bit 2 nt + e of mb[mt] = this lane's accumulator element (mt, nt, e) belongs to an observed sample
             uint32_t mb[MT];
             if constexpr (kMis) {
 #pragma unroll
                 for (int mt = 0; mt < MT; ++mt) {
-                    const unsigned long long* row = P.mbits + (size_t)(k0 + tr0 + mt * 8 + g) * P.mwords;
+                    const unsigned long long* row = P.mbits + (size_t)(k0 + mt * 8 + g) * P.mwords;
                     uint32_t bits = 0;
 #pragma unroll
                     for (int nt = 0; nt < NT; ++nt)
@@ -495,7 +490,9 @@ __global__ void __launch_bounds__(Cfg::kThreads, 1) sweep_kernel(const SweepPara
                     mb[mt] = bits;
                 }
             }
-            auto s_issue = [&](long gbi) {
+            // S phase of block gbi: the split-K DMMAs of S'^T = R^T X_b into the accumulators sa, then the accumulator chains
+            // added, the partials stored and the chain warp told
+            auto s_phase = [&](long gbi) {
                 const int stage = (int)(gbi % kStages);
                 AQ_T0();
                 mbar_wait(&full[stage], (uint32_t)((gbi / kStages) & 1));
@@ -513,9 +510,6 @@ __global__ void __launch_bounds__(Cfg::kThreads, 1) sweep_kernel(const SweepPara
                     for (int mt = 0; mt < MT; ++mt) dmma(sa[mt][kSC - 1][0], sa[mt][kSC - 1][1], acc[mt][nt][1], xb.y);
                 }
                 AQ_T(11);
-            };
-            auto s_finish = [&](long gbi) {
-                AQ_T0();
                 if (gbi > 0) mbar_wait(&sfree[0], (uint32_t)((gbi - 1) & 1));  // the previous block's partials have been read
                 AQ_T(12);
                 double* sp = spart + (size_t)ws * kT * Cfg::kSps + offP;
@@ -530,14 +524,9 @@ __global__ void __launch_bounds__(Cfg::kThreads, 1) sweep_kernel(const SweepPara
                 if (lane == 0) mbar_arrive(&sdone[(gbi & 1) * 4 + smsp]);
                 AQ_T(13);
             };
-            if (P.mode == 0) {
-                s_issue(gb);
-                s_finish(gb);
-            }
+            if (P.mode == 0) s_phase(gb);
             for (int b = un.b0; b < un.b1; ++b, ++gb) {
-                const bool s_next = P.mode == 0 && b + 1 < un.b1;
-                if (s_next) s_issue(gb + 1);
-                if (Cfg::kSFin < 0 && s_next) s_finish(gb + 1);
+                if (P.mode == 0 && b + 1 < un.b1) s_phase(gb + 1);
                 // ---- rank-8 update with -Delta_b
                 const int stage = (int)(gb % kStages);
                 AQ_T0();
@@ -548,7 +537,7 @@ __global__ void __launch_bounds__(Cfg::kThreads, 1) sweep_kernel(const SweepPara
                 AQ_T(14);
                 const double* xt = tiles + stage * Cfg::kTileDoubles;
                 const double* db = dbuf + (size_t)(gb & 1) * kT * kBlk;
-                if (kCl && rank == 0 && !(Cfg::kChainForwards && P.mode == 0)) {
+                if (kCl && rank == 0) {
                     // leader: forward the kT x 8 block of -Delta to every follower, one 16-byte asynchronous DSMEM store per
                     // lane, accounted on the follower's barrier (armed by its reducer warp)
                     constexpr int kV2 = kT * kBlk / 2;
@@ -594,9 +583,7 @@ __global__ void __launch_bounds__(Cfg::kThreads, 1) sweep_kernel(const SweepPara
 #pragma unroll
                         for (int mt = 0; mt < MT; ++mt) dmma(acc[mt][nt1][0], acc[mt][nt1][1], nd[mt][1], x1b);
                     }
-                    if (nt == Cfg::kSFin && s_next) s_finish(gb + 1);   // the S accumulators have drained meanwhile
                 }
-                if (Cfg::kSFin >= NT && s_next) s_finish(gb + 1);
                 if constexpr (kMis) {
                     // keep the residual masked: r_k -= delta (mis_k o x_j)  (src/coreLoop.cpp:132 in sample space)
 #pragma unroll
@@ -629,11 +616,11 @@ __global__ void __launch_bounds__(Cfg::kThreads, 1) sweep_kernel(const SweepPara
                     v.y = acc[mt][nt][1];
                     ss = fma(v.x, v.x, ss);
                     ss = fma(v.y, v.y, ss);
-                    *reinterpret_cast<double2*>(P.resid + (size_t)(k0 + tr0 + mt * 8 + g) * P.ld_resid + ig + nt * 8 + 2 * l) = v;
+                    *reinterpret_cast<double2*>(P.resid + (size_t)(k0 + mt * 8 + g) * P.ld_resid + ig + nt * 8 + 2 * l) = v;
                 }
                 ss += __shfl_xor_sync(0xffffffffu, ss, 1);
                 ss += __shfl_xor_sync(0xffffffffu, ss, 2);
-                if (l == 0) rsqs[ws * kT + tr0 + mt * 8 + g] = ss;
+                if (l == 0) rsqs[ws * kT + mt * 8 + g] = ss;
             }
             const bool last_seg = un.seg == P.nseg - 1;
             asm volatile("bar.sync 1, %0;" ::"n"(Cfg::kMmaWarps * 32) : "memory");
@@ -962,16 +949,6 @@ __global__ void __launch_bounds__(Cfg::kThreads, 1) sweep_kernel(const SweepPara
         // a remote operation, they would sit in its load/store queue on the serial path
         auto publish = [&](long gb, const double (&nd)[kBlk]) {
             double* dblk = dbuf + (size_t)(gb & 1) * kT * kBlk;
-            if constexpr (Cfg::kChainForwards) {
-                if (P.mode == 0 && active) {
-                    for (int r2 = 1; r2 < ncta; ++r2) {
-                        const uint32_t rbar = mapa_u32(&dready[gb & 1], r2);
-#pragma unroll
-                        for (int t = 0; t < kBlk; t += 2)
-                            st_async_v2(mapa_u32(dblk + d_off<kT>(tl, t), r2), nd[t], nd[t + 1], rbar);
-                    }
-                }
-            }
             if (active) {
 #pragma unroll
                 for (int t = 0; t < kBlk; t += 2) {
