@@ -11,7 +11,7 @@ _DP = ctypes.POINTER(ctypes.c_double)
 _IP = ctypes.POINTER(ctypes.c_int32)
 
 EXPORTS = ["aq_last_error", "aq_version", "aq_device_info", "aq_create", "aq_destroy", "aq_dims", "aq_set_order",
-           "aq_set_state", "aq_get_state", "aq_get_residual", "aq_refresh_tables", "aq_sweep", "aq_rowsums_zpart",
+           "aq_set_state", "aq_get_state", "aq_get_residual", "aq_get_tables", "aq_refresh_tables", "aq_sweep", "aq_rowsums_zpart",
            "aq_rowsums_zpart_dev", "aq_launch_count", "aq_last_sweep_ms", "aq_last_ms", "aq_sync", "aq_coreDualLoop",
            "aq_set_missing", "aq_set_state_mis", "aq_sweep_mis", "aq_ppi_count_sum", "aq_ppi_next_above", "aq_ppi_collect",
            "aq_prep_x", "aq_prep_geno", "aq_prep_result", "aq_prep_destroy", "aq_prep_launch_count", "aq_create_prepared",

@@ -662,7 +662,7 @@ int create_impl(aq_ctx** out, int device, int n, int p, int q_local, const doubl
     c->ntiles = (q_local + cfg.k->kT - 1) / cfg.k->kT;
     const size_t pq = (size_t)c->p_pad * c->q_pad;
     c->stage_cols = (int)std::max<size_t>(1, std::min<size_t>((size_t)q_local, ((size_t)256 << 20) / (sizeof(double) * (size_t)p)));
-    c->n_partials = (size_t)((c->q + 255) / 256) * ((c->p + kTabRowsPerBlock - 1) / kTabRowsPerBlock);
+    c->n_partials = (size_t)((c->q + 255) / 256) * tab_row_blocks(c->p);   // one per CTA of the table pass
 #define AQ_ALLOC(ptr, count)                                                              \
     do {                                                                                  \
         cudaError_t e_ = cudaMalloc((void**)&(ptr), sizeof(*(ptr)) * (size_t)(count));    \
@@ -1115,6 +1115,17 @@ int aq_get_residual(aq_ctx* c, double* resid) {
     return AQ_OK;
 }
 
+int aq_get_tables(aq_ctx* c, double* D, double* W, double* I0) {
+    if (!c) return fail(AQ_EINVAL, "NULL context");
+    if (!c->have_tables) return fail(AQ_ESTATE, "aq_get_tables before aq_refresh_tables");
+    AQ_CUDA(cudaSetDevice(c->device));
+    int rc = AQ_OK;
+    if (D && (rc = download_pxq(c, c->dtab, nullptr, 0, D)) != AQ_OK) return rc;
+    if (W && (rc = download_pxq(c, c->wtab, nullptr, 0, W)) != AQ_OK) return rc;
+    if (I0 && (rc = download_pxq(c, c->i0tab, nullptr, 0, I0)) != AQ_OK) return rc;
+    return AQ_OK;
+}
+
 int aq_refresh_tables(aq_ctx* c, const double* theta_vb, const double* zeta_vb, double c_next, double* elbo_b_part) {
     if (!c || !theta_vb || !zeta_vb) return fail(AQ_EINVAL, "aq_refresh_tables: NULL argument");
     if (!(c_next > 0.0)) return fail(AQ_EINVAL, "aq_refresh_tables: c_next must be positive");
@@ -1124,13 +1135,19 @@ int aq_refresh_tables(aq_ctx* c, const double* theta_vb, const double* zeta_vb, 
     AQ_CUDA(cudaMemcpyAsync(c->theta, theta_vb, sizeof(double) * c->p, cudaMemcpyHostToDevice, c->stream));
     AQ_CUDA(cudaMemcpyAsync(c->zeta, zeta_vb, sizeof(double) * c->q, cudaMemcpyHostToDevice, c->stream));
     const int c_is_one = std::fabs(c_next - 1.0) < 1.5e-8;  // isTRUE(all.equal(c, 1)), R/update_vb.R:219
-    dim3 grid((c->q + 255) / 256, (c->p + kTabRowsPerBlock - 1) / kTabRowsPerBlock);
+    const int row_blocks = tab_row_blocks(c->p);
     AQ_CUDA(cudaEventRecord(c->evt0, c->stream));
-    tables_kernel<<<grid, 256, 0, c->stream>>>(c->theta, c->zeta, c->p, c->q, c->q_pad, c_is_one ? 1.0 : std::sqrt(c_next),
-                                               c_is_one, c->gam, c->dtab, c->wtab, c->i0tab, elbo_b_part ? 1 : 0,
-                                               c->partials);
-    AQ_CUDA(cudaGetLastError());
-    c->launches++;
+    for (int rb0 = 0; rb0 < row_blocks; rb0 += kTabMaxGridRows) {   // (one launch for p <= 524,280)
+        dim3 grid((c->q + 255) / 256, std::min(row_blocks - rb0, kTabMaxGridRows));
+        const int j0 = rb0 * kTabRowsPerBlock;
+        const size_t off = (size_t)j0 * c->q_pad;
+        tables_kernel<<<grid, 256, 0, c->stream>>>(c->theta + j0, c->zeta, c->p - j0, c->q, c->q_pad,
+                                                   c_is_one ? 1.0 : std::sqrt(c_next), c_is_one, c->gam + off, c->dtab + off,
+                                                   c->wtab + off, c->i0tab + off, elbo_b_part ? 1 : 0,
+                                                   c->partials + (size_t)rb0 * grid.x);
+        AQ_CUDA(cudaGetLastError());
+        c->launches++;
+    }
     if (elbo_b_part) {
         sum_partials_kernel<<<1, 1024, 0, c->stream>>>(c->partials, c->n_partials, c->scalar);
         AQ_CUDA(cudaGetLastError());

@@ -93,8 +93,14 @@ __global__ void fill_kernel(double* __restrict__ x, size_t nelem, double v) {
 //   D = lq - lp;  at U = sqrt(c) u:  imr1 = phi(U)/Phi(U) (>= -U), imr0 = -phi(U)/(1 - Phi(U)) (<= -U)
 //   W = imr1 - imr0;  I0 = imr0.                             (R/utils.R:172-191, R/update_vb.R:217-234)
 // Optional ELBO-B part (R/elbo.R:19-26): sum gam lp + (1-gam) lq - gam log(gam+eps) - (1-gam) log(1-gam+eps).
-// Grid: blockIdx.y strides over rows j, blockIdx.x * blockDim.x covers traits k (coalesced).
+// Grid: blockIdx.y strides over rows j, blockIdx.x * blockDim.x covers traits k (coalesced); one ELBO partial per CTA.
+// gridDim.y is capped at 65,535, so for p > 524,280 the host launches the pass on slices of at most kTabMaxGridRows row
+// blocks, with theta, the p x q arrays and the partials offset to the slice (one launch below that).
 constexpr int kTabRowsPerBlock = 8;
+constexpr int kTabMaxGridRows = 65535;
+
+// row blocks of the table pass: with the 256-trait column blocks, the number of CTAs over all launches and of ELBO partials
+inline int tab_row_blocks(int p) { return (p + kTabRowsPerBlock - 1) / kTabRowsPerBlock; }
 
 // Everything the table pass needs about the standard normal at one point u, from ONE erfcx, ONE exp, one log and
 // one log1p:  with a = |u|/sqrt2, E = erfcx(a), e2 = exp(-u^2/2):  Q = E e2 / 2 is the tail mass beyond |u|,
@@ -123,7 +129,8 @@ __device__ __forceinline__ NormalPoint normal_point(double u, bool want_logs, bo
         o.log_tail = log(0.5 * E) - 0.5 * u * u;
         o.log_body = log1p(-Q);
     }
-    if (want_ratios) {   // E in [0.01, 1], 1 - Q in [0.5, 1]
+    if (want_ratios) {   // E in (0, 1] falls off like 0.8 / |u|: inside fast_rcp's [2^-100, 2^100] for |u| < 2^99.
+                         // 1 - Q in [0.5, 1]
         o.r_tail = kSqrt2OverPi * fast_rcp(E);
         o.r_body = kInvSqrt2Pi * e2 * fast_rcp(1.0 - Q);
     }

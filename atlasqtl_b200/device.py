@@ -123,6 +123,12 @@ class SweepContext:
                                                ctypes.byref(out) if want_elbo else None))
         return out.value if want_elbo else None
 
+    def get_tables(self, D=True, W=True, I0=True):
+        """The tables of the last refresh_tables (aq_get_tables), p x q_local: D = log(1 - Phi(u)) - log Phi(u), W and I0."""
+        outs = [np.empty((self.p, self.q), order="F") if f else None for f in (D, W, I0)]
+        _lib.check(self._lib.aq_get_tables(self._ctx, *[_lib.dptr(x) for x in outs]))
+        return dict(D=outs[0], W=outs[1], I0=outs[2])
+
     def sweep(self, c, log_sig2_inv_vb, tau_vb, log_tau_vb, sig2_beta_vb):
         vecs = [np.ascontiguousarray(v, dtype=np.float64) for v in (tau_vb, log_tau_vb, sig2_beta_vb)]
         for v in vecs:

@@ -139,6 +139,14 @@ int aq_snapshot_fetch(aq_ctx* ctx, double* gam_vb, double* mu_beta_vb, double* b
 int aq_get_residual(aq_ctx* ctx, double* resid);
 
 /*
+ * The three tables of the last aq_refresh_tables, p x q_local each in R layout (column-major), mainly for tests that pin
+ * the table pass entry by entry: D = log(1 - Phi(u)) - log Phi(u) at u = theta_j + zeta_k (the log-odds the sweep
+ * reads), W = imr1 - imr0 and I0 = imr0 at U = sqrt(c_next) u (U = u when c_next is 1).  Any pointer may be NULL.
+ * AQ_ESTATE before the first aq_refresh_tables.
+ */
+int aq_get_tables(aq_ctx* ctx, double* D, double* W, double* I0);
+
+/*
  * Streaming p x q_local pass after theta_vb / zeta_vb changed
  * (replaces R/atlasqtl_global_local_core.R:61-63 and :293-295):
  *   D    = log(1 - Phi(theta_j + zeta_k)) - log Phi(theta_j + zeta_k)      (the only way the sweep uses the tables)
